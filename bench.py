@@ -158,6 +158,9 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ref-gpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy "
+                         "(float32; see dump_positions for the sample kept of a large output)")
     return ap.parse_args()
 
 
@@ -464,6 +467,55 @@ def make_inputs(torch, dev, samples, C, D, H, W, seed):
     return x, go, g, xl, gol, fl
 
 
+# what one call of the timed path returns, in the order one_sample returns it
+DUMP_NAMES = ("sga_out", "sga_mask", "sga_grad_x", "sga_grad_g0", "sga_grad_g1", "sga_grad_g2", "sga_grad_g3",
+              "lga2_out", "lga2_grad_x", "lga2_grad_f")
+DUMP_ELEMENTS = 1 << 20        # per output: 4 MB of float32, so the ten files stay below 64 MB
+
+
+def dump_positions(per_sample, batch):
+    """Flat positions within one sample kept by --dump-outputs: all of them when the whole output fits in
+    DUMP_ELEMENTS, else the same fixed, seeded sample in every sample of the batch."""
+    k = max(1, DUMP_ELEMENTS // batch)
+    if per_sample <= k:
+        return None
+    import numpy as np
+    return np.unique(np.random.default_rng(0).integers(0, per_sample, k))
+
+
+class OutputDump:
+    """Collects, call by call, the outputs of the last timed step on the device and writes them as DIR/<name>.npy.
+    Positions and buffers are set up before the timed window, so that inside it the dump adds only asynchronous
+    device gathers (ten small launches per call, so that no full-size output outlives its call), and nothing when
+    --dump-outputs is not given."""
+
+    def __init__(self, torch, dev, batch, C, D, H, W):
+        per_sample = dict(zip(DUMP_NAMES, [(C, D, H, W)] * 3 + [(C, 5, H, W)] * 4 + [(D, H, W)] * 2 + [(75, H, W)]))
+        self.bufs, self.shapes, self.pos = {}, {}, {}
+        for name, shape in per_sample.items():
+            numel = 1
+            for d in shape:
+                numel *= d
+            p = dump_positions(numel, batch)
+            self.pos[name] = None if p is None else torch.from_numpy(p).to(dev)
+            self.shapes[name] = (batch,) + (shape if p is None else (len(p),))
+            self.bufs[name] = torch.empty((batch, numel if p is None else len(p)), dtype=torch.float32, device=dev)
+
+    def keep(self, first, outputs):
+        flat = (outputs[0], outputs[1], outputs[2]) + tuple(outputs[3]) + tuple(outputs[4:])
+        for name, t in zip(DUMP_NAMES, flat):
+            n = t.shape[0]
+            t = t.reshape(n, -1)
+            pos = self.pos[name]
+            self.bufs[name][first:first + n].copy_(t if pos is None else t.index_select(1, pos))
+
+    def write(self, path):
+        import numpy as np
+        os.makedirs(path, exist_ok=True)
+        for name, buf in self.bufs.items():
+            np.save(os.path.join(path, name + ".npy"), buf.cpu().numpy().reshape(self.shapes[name]))
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -476,6 +528,8 @@ def run_ours(a):
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     world, rank, local_rank = dist_setup("nccl", dev)
+    if a.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes one rank's outputs; run it with --gpus 1")
     B, C, D, H, W = a.batch, a.channels, a.depth, a.height, a.width
     mine = shard_samples(B, world, rank)
     v_sga, v_lga = B * C * D * H * W, B * D * H * W
@@ -513,11 +567,13 @@ def run_ours(a):
         if record:
             e[4].record()
             phase_events.append(e)
-        return out, gi, gg, y, gx, gf
+        return out, mask, gi, gg, y, gx, gf
 
-    def step(record):
+    def step(record, dump=None):
         for i in range(0, len(mine), cs):
-            one_sample(i, record)
+            outputs = one_sample(i, record)
+            if dump is not None:
+                dump.keep(i, outputs)
 
     def sync_all():
         torch.cuda.synchronize()
@@ -528,17 +584,20 @@ def run_ours(a):
     for _ in range(a.warmup):
         step(False)
     sync_all()
+    dump = OutputDump(torch, dev, len(mine), C, D, H, W) if a.dump_outputs else None   # before the timed window
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
     t0, t1 = ev(), ev()
     t0.record()
-    for _ in range(a.steps):
-        step(True)
+    for k in range(a.steps):
+        step(True, dump if k == a.steps - 1 else None)
     t1.record()
     sync_all()
     ms = t0.elapsed_time(t1)
     clk = clocks.stop() if rank == 0 else None
+    if dump is not None:
+        dump.write(a.dump_outputs)
     ms = max_over_ranks(ms, world, dev)
     done = sum_over_ranks(len(mine), world, dev)       # every sample processed exactly once
     assert int(done) == B, (done, B)
@@ -717,7 +776,7 @@ def run_e2e(torch, dist, world, dev, a, mine, v_sga, v_lga):
                 last_out[0] = torch.cuda.Event()
                 last_out[0].record(s_out)
 
-    steps = max(1, min(a.steps, 2))
+    steps = a.steps
     run(2)                                    # warm-up (allocator, both buffers)
     torch.cuda.synchronize()
     if world > 1:
@@ -785,6 +844,8 @@ def ref_gpu_rate(torch, dev, C, D, H, W):
 
 def main():
     a = parse_args()
+    if a.dump_outputs and (a.config is not None or a.impl != "ours"):
+        raise SystemExit("bench.py: --dump-outputs applies to the headline workload of --impl ours")
     if a.config is not None:
         if a.impl == "reference":
             if int(os.environ.get("RANK", "0")) == 0:

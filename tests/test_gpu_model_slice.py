@@ -2,12 +2,12 @@
 its hot-path modules -- SGABlock (models/GANet_deep.py:249-277: guidance split into four
 (N,C,5,H,W) maps, L1-normalised over dim 2, SGA, BN + ReLU, 3-D conv, residual) feeding a
 DispAgg head (:222-247: 3-D conv to one channel, trilinear upsampling, LGA2, softmin, LGA2,
-L1 normalisation, DisparityRegression) on a GetCostVolume input -- is run twice from the same
-weights: once on ganet_b200.modules, once on test-only autograd wrappers around the UNMODIFIED
-reference CUDA extension (oracle/_ref/GANet*.so) that restate libs/GANet/functions/GANet.py.
+L1 normalisation, DisparityRegression) on a GetCostVolume input -- is run on ganet_b200.modules
+and compared with the same network from the same weights on test-only autograd wrappers around the
+UNMODIFIED reference CUDA extension that restate libs/GANet/functions/GANet.py (that run's results
+are in tests/golden/ref_cuda_values.npz, written by tests/golden/make_golden.py --cuda).
 Outputs must agree to 1e-4 relative and every parameter gradient to 1e-3 (fp32; the disparity map and
 SGA outputs feed max/argmax paths, so this is also a check that masks agree)."""
-import numpy as np
 import pytest
 import torch
 import torch.nn as nn
@@ -15,10 +15,10 @@ import torch.nn.functional as F
 from torch.autograd import Function
 
 from oracle import ref_gpu
-from util import assert_close
+from util import assert_close_to_golden, case_id, golden_values
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not ref_gpu.available(), reason="reference CUDA extension not built")]
+pytestmark = pytest.mark.gpu
+HW = [(12, 20), (32, 48)]                                      # the second runs the TMA kernels
 
 
 class RefSga(Function):
@@ -110,28 +110,39 @@ class SliceNet(nn.Module):
         return ref_disp_regression(v) if self.use_reference else self.reg(v)
 
 
-@pytest.mark.parametrize("hw", [(12, 20), (32, 48)])      # the second runs the TMA kernels
-def test_network_slice_matches_reference_extension(hw):
+def slice_setup(hw):
+    """The network on ganet_b200.modules, seeded weights, and its seeded inputs."""
     torch.manual_seed(0)
     torch.backends.cudnn.benchmark = False
     torch.backends.cudnn.deterministic = True
     H, W = hw
-    mine, ref = SliceNet().cuda(), SliceNet(use_reference=True).cuda()
-    ref.load_state_dict(mine.state_dict())
+    net = SliceNet().cuda()
     left, right = torch.randn(2, 3, H, W, device="cuda"), torch.randn(2, 3, H, W, device="cuda")
     target = torch.rand(2, 2 * H, 2 * W, device="cuda") * 8
-    outs = []
-    for net in (mine, ref):
-        net.train()
-        d = net(left, right)
-        loss = F.smooth_l1_loss(d, target)
-        loss.backward()
-        outs.append((d.detach().cpu().numpy(), float(loss.detach()),
-                     {k: p.grad.detach().cpu().numpy() for k, p in net.named_parameters()}))
-    assert_close(outs[0][0], outs[1][0], 1e-4, "disparity map")
-    assert abs(outs[0][1] - outs[1][1]) <= 1e-5 * max(1.0, abs(outs[1][1]))
+    return net, left, right, target
+
+
+def train_step(net, left, right, target):
+    """One training-mode forward + backward -> disparity map, loss, parameter gradients."""
+    net.train()
+    d = net(left, right)
+    loss = F.smooth_l1_loss(d, target)
+    loss.backward()
+    return d.detach(), float(loss.detach()), {k: p.grad.detach() for k, p in net.named_parameters()}
+
+
+@pytest.mark.parametrize("hw", HW)
+def test_network_slice_matches_reference_extension(hw):
+    ref = golden_values("ref_cuda_values.npz")
+    key = "model_slice/%s/" % case_id(hw)
+    d, loss, grads = train_step(*slice_setup(hw))
+    assert_close_to_golden(d, ref, key + "disparity", 1e-4, what="disparity map")
+    ref_loss = float(ref[key + "loss"][0])
+    assert abs(loss - ref_loss) <= 1e-5 * max(1.0, abs(ref_loss))
     # parameter gradients: the operators agree to 1e-4 each (tests/test_gpu_parity.py); between them and the weights
     # sit torch's atomically accumulated interpolation gradients and cuDNN's backward kernels, whose run-to-run noise
     # alone moves a gradient by ~1e-4 of its scale (a 2e-4 bound was seen to fail at 2.09e-4 on an otherwise green run)
-    for k in outs[1][2]:
-        assert_close(outs[0][2][k], outs[1][2][k], 1e-3, "grad of " + k)
+    assert sorted(k[len(key + "grad/"):] for k in ref
+                  if k.startswith(key + "grad/") and not k.endswith("/scale")) == sorted(grads)
+    for k, t in grads.items():
+        assert_close_to_golden(t, ref, key + "grad/" + k, 1e-3, what="grad of " + k)

@@ -1,8 +1,10 @@
 """GPU parity tests (run on the B200 box): the CUDA path, called through the C ABI,
 against
-  (1) the UNMODIFIED reference CUDA extension (oracle/_ref/GANet*.so): SGA forward
-      values, direction mask and depth arg-max BIT-EXACT; gradients and LGA within
-      the north_star tolerance of 1e-4 relative fp32;
+  (1) the UNMODIFIED reference CUDA extension, through its results on the same seeded
+      inputs (tests/golden/ref_cuda_*, written by tests/golden/make_golden.py --cuda):
+      SGA forward values, direction mask and depth arg-max BIT-EXACT (SHA-256 digests);
+      gradients and LGA within the north_star tolerance of 1e-4 relative fp32 (values at
+      fixed sample positions and each tensor's largest magnitude);
   (2) the CPU oracle (oracle/ganet_oracle.c, fused rounding): same criteria;
   (3) the committed golden vectors (tests/golden/, generated from the reference's
       kernel bodies on the host; unfused rounding, hence tolerance not bit-exactness).
@@ -15,14 +17,24 @@ import torch
 
 from oracle import api as oracle
 from oracle import ref_gpu
-from util import assert_close, lga_inputs, sga_inputs
+from util import (GOLD, assert_close, assert_close_to_golden, case_id, digest, golden_json, golden_values,
+                  lga_inputs, sga_inputs)
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-4          # north_star: 1e-4 relative fp32
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 needs_ref = pytest.mark.skipif(not ref_gpu.available(),
                                reason="oracle/_ref/GANet*.so (reference CUDA extension) not built")
+
+
+@pytest.fixture(scope="module")
+def ref_digests():
+    return golden_json("ref_cuda_digests.json")
+
+
+@pytest.fixture(scope="module")
+def ref_values():
+    return golden_values("ref_cuda_values.npz")
 
 
 def cu(a):
@@ -53,36 +65,36 @@ SGA_SHAPES = [(2, 3, 7, 5, 6), (1, 2, 1, 4, 3), (1, 1, 2, 1, 5), (1, 2, 3, 6, 1)
               (1, 1, 300, 4, 6), (1, 2, 513, 3, 5)]
 
 
-@needs_ref
 @pytest.mark.parametrize("shape", SGA_SHAPES)
-def test_sga_forward_bit_exact_vs_reference_cuda(ops, shape):
+def test_sga_forward_bit_exact_vs_reference_cuda(ops, ref_digests, shape):
     x, g, _ = sga_inputs(shape, seed=1 + sum(shape))
     xt, gt = cu(x), [cu(a) for a in g]
     out, mask = ops.sga_forward(xt, *gt)
-    ro, rm, rtemp = ref_gpu.sga_forward(xt, *gt)
-    torch.cuda.synchronize()
-    assert torch.equal(out, ro), "SGA forward values differ from the reference CUDA kernels"
-    assert torch.equal(mask, rm.to(torch.uint8)), "direction mask differs"
-    assert torch.equal(ops.sga_direction(xt, gt[3], 3), rtemp), "left aggregate differs"
+    key = "sga_forward/%s/" % case_id(shape)
+    assert digest(out) == ref_digests[key + "out"], "SGA forward values differ from the reference CUDA kernels"
+    assert digest(mask, np.uint8) == ref_digests[key + "mask"], "direction mask differs"
+    assert digest(ops.sga_direction(xt, gt[3], 3)) == ref_digests[key + "left"], "left aggregate differs"
 
 
-@needs_ref
+DIRECTION_SHAPE = (1, 2, 12, 20, 24)
+
+
 @pytest.mark.parametrize("direction", [0, 1, 2, 3])
-def test_each_direction_bit_exact_vs_reference_cuda(ops, direction):
+def test_each_direction_bit_exact_vs_reference_cuda(ops, ref_digests, direction):
     """Isolate one scan kernel of the reference: x in [1, 1.1) with positive weights
     keeps every aggregate in [1, 1.1); scaling the guidance of `direction` by 1.2
     lifts that aggregate above 1.2 everywhere, so it wins the max at every voxel and
-    `out` IS that direction's aggregate."""
-    shape = (1, 2, 12, 20, 24)
-    x, g, _ = sga_inputs(shape, seed=40 + direction, positive=True)
+    `out` IS that direction's aggregate (make_golden.py asserts that the reference's
+    mask is `direction` everywhere)."""
+    x, g, _ = sga_inputs(DIRECTION_SHAPE, seed=40 + direction, positive=True)
     g[direction] = (g[direction] * 1.2).astype(np.float32)
     xt, gt = cu(x), [cu(a) for a in g]
-    ro, rm, _ = ref_gpu.sga_forward(xt, *gt)
-    assert bool((rm == direction).all()), "construction failed: direction does not dominate"
+    key = "sga_direction/%d/" % direction
     mine = ops.sga_direction(xt, gt[direction], direction)
-    assert torch.equal(mine, ro)
+    assert digest(mine) == ref_digests[key + "out"]
     out, mask = ops.sga_forward(xt, *gt)
-    assert torch.equal(out, ro) and torch.equal(mask, rm.to(torch.uint8))
+    assert bool((mask == direction).all()), "construction failed: direction does not dominate"
+    assert digest(out) == ref_digests[key + "out"] and digest(mask, np.uint8) == ref_digests[key + "mask"]
 
 
 @pytest.mark.parametrize("shape", SGA_SHAPES)
@@ -96,24 +108,23 @@ def test_sga_forward_bit_exact_vs_oracle(ops, shape):
         assert np.array_equal(npy(ops.sga_direction(cu(x), cu(g[d]), d)), od[d])
 
 
-@needs_ref
 @pytest.mark.parametrize("shape", SGA_SHAPES)
-def test_sga_backward_vs_reference_cuda(ops, shape):
+def test_sga_backward_vs_reference_cuda(ops, ref_digests, ref_values, shape):
     x, g, go = sga_inputs(shape, seed=3 + sum(shape))
     xt, gt, got = cu(x), [cu(a) for a in g], cu(go)
-    ro, rm, rtemp = ref_gpu.sga_forward(xt, *gt)
-    rgi, rgg, ridx = ref_gpu.sga_backward(xt, *gt, rtemp, rm, got)
     out, mask = ops.sga_forward(xt, *gt)
     gi, gg, idx = ops.sga_backward(xt, *gt, mask, got, want_max_idx=True)
-    torch.cuda.synchronize()
-    assert torch.equal(idx, ridx.to(torch.int32)), "max_idx (depth arg-max) differs"
-    assert_close(npy(gi), npy(rgi), RTOL, "gradInput")
+    key = "sga_backward/%s/" % case_id(shape)
+    assert digest(idx, np.int32) == ref_digests[key + "idx"], "max_idx (depth arg-max) differs"
+    assert_close_to_golden(gi, ref_values, key + "gi", RTOL, what="gradInput")
     for d in range(4):
-        assert_close(npy(gg[d]), npy(rgg[d]), RTOL, "guidance grad %d" % d)
+        assert_close_to_golden(gg[d], ref_values, key + "gg%d" % d, RTOL, what="guidance grad %d" % d)
 
 
-@pytest.mark.parametrize("shape", SGA_SHAPES[:8] + SGA_SHAPES[12:15])
+@pytest.mark.parametrize("shape", SGA_SHAPES)
 def test_sga_backward_vs_oracle(ops, shape):
+    """Every element of every gradient against the CPU oracle (pinned to the reference's kernel bodies by
+    test_oracle.py), including the D > 288 shapes that exercise the generic line-kernel backward."""
     x, g, go = sga_inputs(shape, seed=4 + sum(shape))
     xt, gt = cu(x), [cu(a) for a in g]
     out, mask = ops.sga_forward(xt, *gt)
@@ -295,21 +306,19 @@ LGA_SHAPES = [(2, 7, 5, 6), (1, 3, 9, 11), (1, 1, 1, 1), (1, 5, 1, 40), (1, 4, 3
               (1, 9, 12, 40), (2, 6, 9, 44), (1, 33, 20, 152), (1, 4, 8, 72), (2, 2, 5, 8, 40)]
 
 
-@needs_ref
 @pytest.mark.parametrize("shape", LGA_SHAPES)
-def test_lga2_vs_reference_cuda(ops, shape):
+def test_lga2_vs_reference_cuda(ops, ref_values, shape):
     x, f, go = lga_inputs(shape, seed=5)
     xt, ft, got = cu(x), cu(f), cu(go)
-    ry, ry1 = ref_gpu.lga2_forward(xt, ft)
-    rgx, rgf = ref_gpu.lga2_backward(xt, ft, ry1, got)
     y1 = ops.lga_forward(xt, ft, 2)
     y = ops.lga_forward(y1, ft, 2)
     g1, gf = ops.lga_backward(y1, ft, got, 2)
     gx, gf = ops.lga_backward(xt, ft, g1, 2, grad_f=gf)
-    assert_close(npy(y1), npy(ry1), RTOL, "y1")
-    assert_close(npy(y), npy(ry), RTOL, "y")
-    assert_close(npy(gx), npy(rgx), RTOL, "grad_x")
-    assert_close(npy(gf), npy(rgf), RTOL, "grad_f")
+    key = "lga2/%s/" % case_id(shape)
+    assert_close_to_golden(y1, ref_values, key + "y1", RTOL, what="y1")
+    assert_close_to_golden(y, ref_values, key + "y", RTOL, what="y")
+    assert_close_to_golden(gx, ref_values, key + "gx", RTOL, what="grad_x")
+    assert_close_to_golden(gf, ref_values, key + "gf", RTOL, what="grad_f")
 
 
 @pytest.mark.parametrize("shape", LGA_SHAPES)
@@ -459,9 +468,11 @@ def test_disparity_regression_at_model_shapes(shape):
              e[1].elapsed_time(e[2]) / 10, nb / (e[1].elapsed_time(e[2]) / 10) / 1e6))
 
 
-@needs_ref
-@pytest.mark.parametrize("fname,passes", [("LgaFunction", 1), ("Lga3Function", 3), ("Lga3d3Function", 3)])
-def test_lga_1_and_3_pass_functions_through_autograd(fname, passes):
+LGA_PASSES = [("LgaFunction", 1), ("Lga3Function", 3), ("Lga3d3Function", 3)]
+
+
+@pytest.mark.parametrize("fname,passes", LGA_PASSES)
+def test_lga_1_and_3_pass_functions_through_autograd(ref_values, fname, passes):
     """LgaFunction / Lga3Function (broken upstream: functions/GANet.py:155,241-242) and Lga3d3Function
     through torch.autograd on the GPU, against `passes` chained calls of the reference extension's
     lga_cuda_forward / backward with its accumulate-into-gradFilters contract."""
@@ -472,15 +483,10 @@ def test_lga_1_and_3_pass_functions_through_autograd(fname, passes):
     xt, ft = cu(x).requires_grad_(), cu(f).requires_grad_()
     y = fn.apply(xt, ft, 2)
     y.backward(cu(go))
-    xs = [cu(x)]
-    for _ in range(passes):
-        xs.append(ref_gpu.lga_forward(xs[-1], cu(f), 2))
-    assert_close(npy(y), npy(xs[-1]), RTOL, fname + " output")
-    g, gf = cu(go), None
-    for k in range(passes - 1, -1, -1):
-        g, gf = ref_gpu.lga_backward(xs[k], cu(f), g, gf, 2)
-    assert_close(npy(xt.grad), npy(g), RTOL, fname + " grad_x")
-    assert_close(npy(ft.grad), npy(gf), RTOL, fname + " grad_filters")
+    key = "lga_passes/%s/" % fname
+    assert_close_to_golden(y, ref_values, key + "y", RTOL, what=fname + " output")
+    assert_close_to_golden(xt.grad, ref_values, key + "gx", RTOL, what=fname + " grad_x")
+    assert_close_to_golden(ft.grad, ref_values, key + "gf", RTOL, what=fname + " grad_filters")
 
 
 # ---- autograd / API behaviour -----------------------------------------------------
@@ -566,7 +572,6 @@ def test_cuda_graph_capture_and_replay(ops):
         assert_close(npy(gg[d]), ogg[d], RTOL, "guidance grad")
 
 
-@needs_ref
 def _pybind_module():
     import glob
     import importlib.util
@@ -580,9 +585,31 @@ def _pybind_module():
     return mod
 
 
-@needs_ref
+def run_legacy_surface(mod):
+    """SGA forward + backward through a module with the reference's native surface, buffers as the
+    reference's Python layer allocates them -> out, temp, mask, gradInput, guidance grads, max_idx."""
+    shape = (1, 2, 6, 5, 7)
+    x, g, go = sga_inputs(shape, seed=15)
+    xt, gt, got = cu(x), [cu(a) for a in g], cu(go)
+    out, temp, mask = (torch.zeros_like(xt) for _ in range(3))
+    assert mod.sga_cuda_forward(xt, *gt, temp, out, mask) == 1
+    gi, tg = torch.zeros_like(xt), torch.zeros_like(xt)
+    gg = [torch.zeros_like(gt[0]) for _ in range(4)]
+    idx = torch.zeros(shape[0], shape[1], shape[3], shape[4], device="cuda")
+    assert mod.sga_cuda_backward(xt, *gt, temp.clone(), mask, idx, got, tg, gi, *gg) == 1
+    return out, temp, mask, gi, gg, idx
+
+
+def run_legacy_lga(mod):
+    xl, fl, _ = lga_inputs((1, 5, 6, 7), seed=16)
+    xl, fl = cu(xl), cu(fl)
+    y = torch.zeros_like(xl)
+    mod.lga_cuda_forward(xl, fl, y, 2)
+    return y
+
+
 @pytest.mark.parametrize("surface", ["legacy_native", "pybind"])
-def test_legacy_native_surface_matches_reference_extension(surface):
+def test_legacy_native_surface_matches_reference_extension(ref_digests, ref_values, surface):
     """The reference's native module surface -- as Python adapters (ganet_b200.legacy_native) and as the
     compiled pybind11 module `GANet` (csrc/ganet_pybind.cpp) -- honours the reference's buffer contract
     (caller-zeroed buffers, accumulate, fp32 mask, temp_out = left aggregate)."""
@@ -590,32 +617,14 @@ def test_legacy_native_surface_matches_reference_extension(surface):
         mine = _pybind_module()
     else:
         from ganet_b200 import legacy_native as mine
-    ref = ref_gpu.module()
-    shape = (1, 2, 6, 5, 7)
-    x, g, go = sga_inputs(shape, seed=15)
-    xt, gt, got = cu(x), [cu(a) for a in g], cu(go)
-
-    def run(mod):
-        out, temp, mask = (torch.zeros_like(xt) for _ in range(3))
-        assert mod.sga_cuda_forward(xt, *gt, temp, out, mask) == 1
-        gi, tg = torch.zeros_like(xt), torch.zeros_like(xt)
-        gg = [torch.zeros_like(gt[0]) for _ in range(4)]
-        idx = torch.zeros(shape[0], shape[1], shape[3], shape[4], device="cuda")
-        assert mod.sga_cuda_backward(xt, *gt, temp.clone(), mask, idx, got, tg, gi, *gg) == 1
-        return out, temp, mask, gi, gg, idx
-
-    a, b = run(mine), run(ref)
-    assert torch.equal(a[0], b[0]) and torch.equal(a[1], b[1]) and torch.equal(a[2], b[2])
-    assert torch.equal(a[5], b[5])
-    assert_close(npy(a[3]), npy(b[3]), RTOL, "gradInput")
-    for p, q in zip(a[4], b[4]):
-        assert_close(npy(p), npy(q), RTOL, "guidance grad")
-    xl, fl, gol = lga_inputs((1, 5, 6, 7), seed=16)
-    xl, fl, gol = cu(xl), cu(fl), cu(gol)
-    ya, yb = torch.zeros_like(xl), torch.zeros_like(xl)
-    mine.lga_cuda_forward(xl, fl, ya, 2)
-    ref.lga_cuda_forward(xl, fl, yb, 2)
-    assert_close(npy(ya), npy(yb), RTOL, "lga forward")
+    a = run_legacy_surface(mine)
+    for k, t in zip(("out", "temp", "mask"), a[:3]):
+        assert digest(t) == ref_digests["legacy_surface/" + k], k
+    assert digest(a[5]) == ref_digests["legacy_surface/idx"]
+    assert_close_to_golden(a[3], ref_values, "legacy_surface/gi", RTOL, what="gradInput")
+    for d in range(4):
+        assert_close_to_golden(a[4][d], ref_values, "legacy_surface/gg%d" % d, RTOL, what="guidance grad")
+    assert_close_to_golden(run_legacy_lga(mine), ref_values, "legacy_surface/lga", RTOL, what="lga forward")
 
 
 @needs_ref

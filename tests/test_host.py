@@ -131,25 +131,19 @@ def test_reference_import_surface():
         assert callable(getattr(G2, name))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference tree not present")
 def test_reference_models_construct_unchanged():
-    """models/GANet_deep.py and GANet11.py import and build on the new modules; the
-    parameter counts are the reference's (SURVEY.md Appendix C.4)."""
-    sys.path.append("/root/reference")
-    try:
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-            del sys.modules[k]
-        from models.GANet_deep import GANet as Deep
-        from models.GANet11 import GANet as G11
-        deep, g11 = Deep(192), G11(192)
-        assert sum(p.numel() for p in deep.parameters()) == 6580112
-        assert sum(p.numel() for p in g11.parameters()) == 4483728
-        assert len(deep.state_dict()) == 479 and len(g11.state_dict()) == 364
-        import ganet_b200.modules as M
-        assert isinstance(deep.cost_agg.sga1.SGA, M.SGA)
-        assert isinstance(deep.cv, M.GetCostVolume)
-    finally:
-        sys.path.remove("/root/reference")
+    """models/GANet_deep.py and GANet11.py (as copied by oracle/build_ref.py into baseline/_ref/models)
+    import and build on the new modules; the parameter counts are the reference's (SURVEY.md Appendix C.4)."""
+    from baseline import refmodels
+    if not refmodels.available():
+        pytest.skip("baseline/_ref/models not built (no reference tree at build time)")
+    deep, g11 = refmodels.build("GANet_deep", 192), refmodels.build("GANet11", 192)
+    assert sum(p.numel() for p in deep.parameters()) == 6580112
+    assert sum(p.numel() for p in g11.parameters()) == 4483728
+    assert len(deep.state_dict()) == 479 and len(g11.state_dict()) == 364
+    import ganet_b200.modules as M
+    assert isinstance(deep.cost_agg.sga1.SGA, M.SGA)
+    assert isinstance(deep.cv, M.GetCostVolume)
 
 
 def _ref_myloss2(input1, input2, thresh=1, alpha=2):
@@ -227,6 +221,38 @@ def test_bench_samples_per_call():
     assert bench.samples_per_call(4, 8, lambda c: c <= 2) == 2
     assert bench.samples_per_call(2, 0, lambda c: False) == 1         # a rank without samples
     assert bench.samples_per_call(3, 8, lambda c: False) == 1
+
+
+def test_bench_output_dump(tmp_path, monkeypatch):
+    """--dump-outputs: one float32 file per output of the timed path, filled call by call at the caller's batch
+    offset; an output larger than its share of DUMP_ELEMENTS is kept at the same seeded positions in every sample,
+    chosen when the dump is set up (before the timed window)."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_ELEMENTS", 200)
+    B, C, D, H, W = 3, 2, 4, 3, 5
+    gen = torch.Generator().manual_seed(0)
+
+    def outputs(n):
+        out = torch.randn(n, C, D, H, W, generator=gen)
+        return (out, (out > 0).to(torch.uint8), -out, [torch.randn(n, C, 5, H, W, generator=gen) for _ in range(4)],
+                torch.randn(n, D, H, W, generator=gen), torch.randn(n, D, H, W, generator=gen),
+                torch.randn(n, 75, H, W, generator=gen))
+
+    first, second = outputs(2), outputs(1)
+    dump = bench.OutputDump(torch, "cpu", B, C, D, H, W)
+    dump.keep(0, first)
+    dump.keep(2, second)
+    dump.write(str(tmp_path))
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(n + ".npy" for n in bench.DUMP_NAMES)
+    pos = bench.dump_positions(C * D * H * W, B)
+    assert pos is not None and np.array_equal(pos, bench.dump_positions(C * D * H * W, B))
+    out = np.load(tmp_path / "sga_out.npy")
+    assert out.dtype == np.float32 and out.shape == (B, len(pos))
+    assert np.array_equal(out[:2], first[0].reshape(2, -1)[:, pos].numpy())
+    assert np.array_equal(out[2], second[0].reshape(-1)[pos].numpy())
+    assert np.array_equal(np.load(tmp_path / "sga_mask.npy"), (out > 0).astype(np.float32))
+    y = np.load(tmp_path / "lga2_out.npy")                      # small enough to keep whole
+    assert y.shape == (B, D, H, W) and np.array_equal(y, torch.cat([first[4], second[4]]).numpy())
 
 
 def test_reference_arm_prints_one_contract_line():

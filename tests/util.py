@@ -1,5 +1,95 @@
-"""Shared input generators for the tests (numpy side and torch side)."""
+"""Shared input generators for the tests (numpy side and torch side), and access to the golden files
+that hold the reference implementation's results (tests/golden/make_golden.py writes them)."""
+import hashlib
+import json
+import os
+
 import numpy as np
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+FULL = 2048           # a tensor compared within a tolerance is kept whole up to this many elements,
+SAMPLE = 1024         # else at (at least) this many positions, every index of every axis among them
+
+
+def golden_json(name):
+    with open(os.path.join(GOLD, name)) as fh:
+        return json.load(fh)
+
+
+def golden_values(name):
+    """A golden file of tolerance records as {key: values at sample_positions, key + "/scale": max |t|}.  The
+    file packs every record into one array (keys, offsets, values, scales): see pack_golden_values."""
+    z = np.load(os.path.join(GOLD, name))
+    out = {}
+    for k, lo, hi, s in zip(z["keys"], z["offsets"][:-1], z["offsets"][1:], z["scales"]):
+        out[str(k)] = z["values"][lo:hi]
+        out[str(k) + "/scale"] = float(s)
+    return out
+
+
+def pack_golden_values(path, records):
+    """Write {key: (values, scale)} in the layout golden_values reads."""
+    keys = sorted(records)
+    vals = [np.asarray(records[k][0], np.float32).reshape(-1) for k in keys]
+    np.savez_compressed(path, keys=np.array(keys), offsets=np.cumsum([0] + [v.size for v in vals]),
+                        values=np.concatenate(vals), scales=np.array([records[k][1] for k in keys], np.float64))
+
+
+def case_id(shape):
+    return "x".join(map(str, shape))
+
+
+def digest(a, dtype=np.float32):
+    """SHA-256 of an array's values as `dtype`, C order: how a golden file pins a result that must match bit
+    for bit without storing it.  Takes numpy arrays and torch tensors (copied to the host)."""
+    if hasattr(a, "detach"):
+        a = a.detach().cpu().numpy()
+    return hashlib.sha256(np.ascontiguousarray(np.asarray(a).astype(dtype, copy=False)).tobytes()).hexdigest()
+
+
+def sample_positions(shape):
+    """Fixed flat positions at which a golden file keeps a tensor of this shape: all of them up to FULL
+    elements, else max(SAMPLE, largest dimension) seeded positions whose coordinates along every axis run
+    through every index of that axis (each about equally often), so that an error confined to one slice --
+    the last depth plane, say -- is among the positions."""
+    shape = tuple(int(d) for d in shape)
+    n = int(np.prod(shape))
+    if n <= FULL:
+        return np.arange(n)
+    k = max(SAMPLE, max(shape))
+    rng = np.random.default_rng(n)
+    coords = [rng.permutation(np.resize(np.arange(d), k)) for d in shape]
+    return np.unique(np.ravel_multi_index(coords, shape))
+
+
+def sampled(t):
+    """(values at sample_positions, max |t|) of a numpy array or torch tensor; a device tensor is gathered on
+    the device, so only the sample is copied."""
+    if hasattr(t, "detach"):
+        import torch
+        flat = t.detach().reshape(-1)
+        pos = torch.from_numpy(sample_positions(t.shape)).to(flat.device)
+        return (flat.index_select(0, pos).float().cpu().numpy(),
+                float(flat.abs().max()) if flat.numel() else 0.0)
+    t = np.asarray(t, np.float32)
+    flat = t.reshape(-1)
+    return flat[sample_positions(t.shape)], float(np.abs(flat).max()) if flat.size else 0.0
+
+
+def assert_close_to_golden(a, gold, key, rtol=1e-4, atol=None, what=""):
+    """assert_close against a reference tensor of which the golden file `gold` keeps the values at
+    sample_positions (`key`) and the largest magnitude (`key/scale`): the per-tensor relative error and the
+    element-wise allclose on the kept positions, and the largest magnitudes within the same bound.
+    atol defaults to rtol * scale, as in assert_close."""
+    vals, amax = sampled(a)
+    ref, scale = gold[key], float(gold[key + "/scale"])
+    what = what or key
+    assert vals.shape == ref.shape, (what, vals.shape, ref.shape)
+    s = max(scale, 1e-30)
+    assert abs(amax - scale) <= rtol * s, "%s: max |a| %.9g vs the reference's %.9g" % (what, amax, scale)
+    err = float(np.abs(vals.astype(np.float64) - ref).max()) / s if vals.size else 0.0
+    assert err <= rtol, "%s: relative error %.3g > %.1g" % (what, err, rtol)
+    assert np.allclose(vals, ref, rtol=rtol, atol=rtol * s if atol is None else atol * s), what
 
 
 def l1norm(a, axis):
